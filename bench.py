@@ -4,6 +4,11 @@ plus the roofline of the dominant kernel and the CPU baseline, as ONE JSON line 
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config 7b|13b-int3|65b|prefill]   # our arm
     python bench.py --impl reference [--steps K] [--warmup W]                                  # the reference's arithmetic on the host cores
+    ... --dump-outputs DIR   # also write what the timed path computed in its last step as DIR/<name>.npy
+
+The inputs are seeded, so two builds run with the same arguments can be compared output for output.  Compare the decode outputs with a
+tolerance: the persistent kernel combines split-K partial sums with unordered fp32 atomics, so even one build differs from run to run by
+fp16 rounding noise (DESIGN.md, run-to-run spread; on a B200 at 1000 W, 32 layers: logits within 0.023 of an rms of 1.29, same greedy token).
 
 A "step" is one decoded token: one replay of the captured CUDA graph of gptq_llama_decode_step (ONE persistent kernel) over a
 random-init LLaMA-7B-shaped GPTQ model (32 distinct layers, 3.6 GB of packed weights per step, i.e. far larger than the 126 MB
@@ -56,6 +61,19 @@ CONFIGS = {  # name -> (size, bits, act_order, BASELINE.json config)
     '65b-tp': ('65b', 4, False, 'LLaMA-65B int4 g128 batch=1 decode, tensor-parallel over the N GPUs (BASELINE config 5)'),
 }
 GROUP = 128
+DUMP_LIMIT_BYTES = 64 << 20
+PREFILL_DUMP_ROWS = 256  # seeded sample of the M = 65536 prefill rows that --dump-outputs writes
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each tensor as <out_dir>/<name>.npy: integers as float64 (exact), everything else as float32."""
+    import numpy as np
+    conv = {k: v.detach().cpu().numpy().astype(np.float32 if v.is_floating_point() else np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in conv.values())
+    assert total <= DUMP_LIMIT_BYTES, f'outputs to dump are {total} bytes, more than {DUMP_LIMIT_BYTES}'
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in conv.items():
+        np.save(os.path.join(out_dir, k + '.npy'), a)
 
 
 def alg_bytes_qlinear(K, N, bits, M=1, gs=GROUP):
@@ -114,7 +132,7 @@ class CpuToken:
         ts = []
         for _ in range(steps):
             t0 = time.perf_counter()
-            self.token()
+            self.logits = self.token()
             ts.append(time.perf_counter() - t0)
         return ts
 
@@ -129,7 +147,7 @@ def cpu_baseline(steps=2, warmup=1):
         'value': 1.0 / t, 'unit': 'tokens/s', 'cores': threads, 'kind': 'port',
         'sample': f'oracle {c.kind} restatement of matmul_248 / fusedmatmul_248 on {threads} host threads: {steps} WHOLE decoded tokens (32 layers x 5 quantized linears at '
                   f'M=1 + attention over 2047 cached tokens + fp16 lm_head), median {t:.2f} s/token; one layer\'s tensors reused for all 32 layers',
-    }, ts
+    }, ts, c.logits
 
 
 def cpu_baseline_subprocess(steps=3, warmup=1):
@@ -150,14 +168,16 @@ def run_reference(args):
     if rank != 0:
         return
     torch.set_num_threads(int(os.environ['OMP_NUM_THREADS']))
-    steps = min(max(1, args.steps), 8)  # bounded sample: a few seconds per token
+    steps = args.steps  # a few seconds per token
     warm = min(max(0, args.warmup), 1)
-    base, ts = cpu_baseline(steps, warm)
+    base, ts, logits = cpu_baseline(steps, warm)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {'logits': logits})
     line = {
         'impl': 'reference', 'metric': METRIC, 'value': base['value'], 'unit': 'tokens/s', 'n_gpus': args.gpus, 'steps': steps, 'warmup': warm,
         'ms_per_step': statistics.mean(ts) * 1e3, 'higher_is_better': True, 'scaling': 'weak', 'vs_baseline': None, 'dtype': 'f16', 'data': 'synthetic',
         'config': {'workload': f'LLaMA-7B int4 g128 batch=1 decode, context {SEQ - 1} (seq={SEQ}), 32 layers, random-init packed weights',
-                   'note': f'CPU arm: steps bounded to {steps} whole tokens (requested {args.steps}); same workload as the GPU arm'},
+                   'note': f'CPU arm: {steps} whole tokens; same workload as the GPU arm'},
         'cpu_baseline': base,
         'e2e': {'value': base['value'], 'unit': 'tokens/s', 'h2d_bytes_per_step': 0, 'd2h_bytes_per_step': 0},
         'gpu_launches': 0,
@@ -235,15 +255,16 @@ def run_decode(args):
     from gptq_b200 import engine, ops
 
     size, bits, act, title = CONFIGS[args.config]
-    steps, warm = max(1, args.steps), max(3, args.warmup)
+    steps, warm = args.steps, max(3, args.warmup)
     tp = args.config.endswith('-tp') and world > 1  # ONE sequence sharded over the ranks (strong scaling) instead of one replica per rank
     if tp:
         dec = engine.synthetic_llama_tp(size, rank, world, bits=bits, groupsize=GROUP, device=str(dev), seed=0, max_seq=SEQ)
     else:
         dec = engine.synthetic_llama(size, bits=bits, groupsize=GROUP, act_order=act, device=str(dev), seed=rank, max_seq=SEQ)
     # synthetic context: the cache holds seq-1 = 2047 tokens of random K/V; the step decodes token 2048
-    dec.k_cache.normal_(0, 0.5)
-    dec.v_cache.normal_(0, 0.5)
+    gen = torch.Generator(device=dev).manual_seed(1000 + rank)
+    dec.k_cache.normal_(0, 0.5, generator=gen)
+    dec.v_cache.normal_(0, 0.5, generator=gen)
     pos = SEQ - 1
     dec.positions.fill_(pos)
     dec.tokens.fill_(1)
@@ -255,6 +276,10 @@ def run_decode(args):
     assert bool(torch.isfinite(dec.logits).all()), 'non-finite logits'
     sampler = ClockSampler(local) if rank == 0 else None
     t_dev = timed(dec.step, steps, dist_on)
+    # what the caller of the last timed step receives: logits, the greedy next token, and the K/V the step wrote at `pos` of every layer
+    # (taken now: the end-to-end arm below feeds the tokens it picks back in)
+    outputs = {'logits': dec.logits.float().cpu(), 'next_tokens': dec.next_tokens.cpu(), 'k_cache_at_pos': dec.k_cache[:, :, :, pos].float().cpu(),
+               'v_cache_at_pos': dec.v_cache[:, :, :, pos].float().cpu()} if args.dump_outputs else None
 
     # ---- end-to-end arm: host token in -> H2D -> step -> D2H logits, every step -----------------------
     tok_host = torch.ones(1, dtype=torch.int32).pin_memory()
@@ -352,6 +377,8 @@ def run_decode(args):
                 pass
         if base is not None:
             line['cpu_baseline'] = base
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     if dist_on:
         dist.destroy_process_group()
@@ -369,18 +396,23 @@ def run_prefill(args):
     t4 = lambda w: (w.qweight, w.scales, w.qzeros, w.g_idx)
     x = torch.randn(M, H, device=dev, generator=gen).half()
 
-    def layer():
-        ops.matmul248(x, *t4(L['qkv']), 4, None, groupsize=GROUP)
-        ops.matmul248(x, *t4(L['o']), 4, None, groupsize=GROUP)
-        h = ops.fused_mlp(x, t4(L['gate']), t4(L['up']), 4, GROUP)
-        ops.matmul248(h, *t4(L['down']), 4, None, groupsize=GROUP)
+    out = {}
 
-    steps, warm = max(1, min(args.steps, 20)), max(3, min(args.warmup, 5))
+    def layer():
+        out['qkv'] = ops.matmul248(x, *t4(L['qkv']), 4, None, groupsize=GROUP)
+        out['o'] = ops.matmul248(x, *t4(L['o']), 4, None, groupsize=GROUP)
+        out['mlp'] = ops.fused_mlp(x, t4(L['gate']), t4(L['up']), 4, GROUP)
+        out['down'] = ops.matmul248(out['mlp'], *t4(L['down']), 4, None, groupsize=GROUP)
+
+    steps, warm = args.steps, max(3, min(args.warmup, 5))
     for _ in range(warm):
         layer()
     sampler = ClockSampler(dev.index)
     t = timed(layer, steps, False) / steps
     clocks = sampler.stop()
+    if args.dump_outputs:  # the four outputs of the last step on a seeded sample of PREFILL_DUMP_ROWS of the M rows
+        rows = torch.randperm(M, generator=torch.Generator().manual_seed(0))[:PREFILL_DUMP_ROWS].sort().values.to(dev)
+        dump_outputs(args.dump_outputs, {'rows': rows, **{k: v.index_select(0, rows).float() for k, v in out.items()}})
     flops = 2 * M * (H * 3 * H + H * H + 2 * H * I + I * H)
     _, burst, sustained, src = measured_peaks()
     print(json.dumps({
@@ -401,7 +433,10 @@ def main():
     ap.add_argument('--warmup', type=int, default=10)
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     ap.add_argument('--config', default='7b', choices=sorted(CONFIGS) + ['prefill'])
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write what the timed path computed in its last step as DIR/<name>.npy (float32 / float64)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.impl == 'reference':
         run_reference(args)
     elif args.config == 'prefill':

@@ -113,6 +113,56 @@ def test_load_quant_style_surgery_on_hf_llama():
     assert quant.autotune_warmup_linear(model) == 0 and quant.autotune_warmup_fused(model) == 0  # nothing on the GPU yet
 
 
+def test_load_quant_recipe_routes_checkpoint_tensors(tmp_path):
+    """A GPTQ checkpoint saved from a make_quant_linear model and loaded the way llama_inference.load_quant loads one (fresh fp16 model,
+    make_quant_linear without lm_head, non-strict load, then attention / norm / MLP fusion and warm-up): every tensor arrives where the
+    kernels read it."""
+    from transformers import LlamaConfig, LlamaForCausalLM
+    cfg = LlamaConfig(hidden_size=256, intermediate_size=768, num_hidden_layers=2, num_attention_heads=2, num_key_value_heads=2, vocab_size=320,
+                      max_position_embeddings=64, rms_norm_eps=1e-6)
+
+    def quant_model():
+        torch.set_default_dtype(torch.half)
+        try:
+            m = LlamaForCausalLM(cfg).eval()
+        finally:
+            torch.set_default_dtype(torch.float)
+        layers = utils.find_layers(m)
+        del layers['lm_head']
+        quant.make_quant_linear(m, layers, 4, 128)
+        return m
+
+    src = quant_model()
+    g = torch.Generator().manual_seed(0)
+    for m in src.modules():
+        if isinstance(m, quant.QuantLinear):
+            m.qweight.copy_(torch.randint(-2**31, 2**31 - 1, m.qweight.shape, generator=g, dtype=torch.int64).to(torch.int32))
+            m.qzeros.copy_(torch.randint(-2**31, 2**31 - 1, m.qzeros.shape, generator=g, dtype=torch.int64).to(torch.int32))
+            m.scales.copy_((torch.rand(m.scales.shape, generator=g) * 1e-2 + 1e-3).half())
+    sd = src.state_dict()
+    assert sd['model.layers.0.self_attn.q_proj.qweight'].shape == (256 // 8, 256) and sd['model.layers.0.mlp.down_proj.qzeros'].dtype == torch.int32
+    ckpt = tmp_path / 'tiny-4bit-128g.pt'
+    torch.save(sd, ckpt)
+
+    model = quant_model()
+    model.load_state_dict(torch.load(ckpt), strict=False)
+    quant.make_quant_attn(model)
+    quant.make_quant_norm(model)
+    quant.make_fused_mlp(model)
+    quant.autotune_warmup_linear(model, transpose=False)
+    quant.autotune_warmup_fused(model)
+    layer = model.model.layers[0]
+    assert isinstance(layer.self_attn, quant.QuantLlamaAttention) and isinstance(layer.mlp, quant.QuantLlamaMLP)
+    assert isinstance(layer.input_layernorm, quant.TritonLlamaRMSNorm) and isinstance(model.model.norm, quant.TritonLlamaRMSNorm)
+    # fused q|k|v along N, gate/up buffers of the fused MLP, down_proj untouched, lm_head never quantized
+    q, k, v = (sd[f'model.layers.0.self_attn.{n}_proj.qweight'] for n in 'qkv')
+    assert torch.equal(layer.self_attn.qkv_proj.qweight, torch.cat([q, k, v], dim=1))
+    assert torch.equal(layer.mlp.gate_proj_qweight, sd['model.layers.0.mlp.gate_proj.qweight'])
+    assert torch.equal(layer.mlp.up_proj_scales, sd['model.layers.0.mlp.up_proj.scales'])
+    assert torch.equal(layer.mlp.down_proj.qzeros, sd['model.layers.0.mlp.down_proj.qzeros'])
+    assert torch.equal(model.lm_head.weight, sd['lm_head.weight'])
+
+
 def test_fuse_qkv_rejects_mismatched_act_order():
     from quant.fused_attn import fuse_qkv
     q, k, v = (quant.QuantLinear(4, 32, 64, 64, False) for _ in range(3))
